@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- genes/s of the full deseq2() hot path (dispersion + IRLS + Wald) on B200, next to the CPU path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -21,6 +21,10 @@ Prints ONE JSON line (rank 0).  `value` = device-resident throughput (counts alr
 CUDA events on the library's stream, L2 flushed between steps, max over ranks.  `e2e` = the same metric through the
 reference-facing plugin calls with HOST buffers (H2D/D2H inside the timed region; page-locked and pageable variants).
 `roofline` describes the dominant kernel, `cpu_baseline` the oracle port (joblib over genes, like the reference).
+
+Every timed loop on the device runs exactly K steps, as does the reference arm; the device arm's `cpu_baseline` is a fixed
+three passes.  `--dump-outputs DIR` writes what the last timed step of the headline workload returned (rank 0's shard) as
+DIR/<name>.npy in float64; the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -50,7 +54,7 @@ KERNEL_OF = {"alpha_mle_genewise": "k_alpha_mle", "alpha_mle_map": "k_alpha_mle"
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of every device measurement and of the reference arm (cpu_baseline: a fixed 3 passes)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--genes", type=int, default=20000)
@@ -61,7 +65,30 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra-configs", action="store_true", help="skip the `configs` block (C3 / C5 shard / C4 shard)")
     ap.add_argument("--lanes", type=int, default=0, help="lanes per gene override (0 = auto)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the arrays the last timed step of the headline workload returned as DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(out_dir, res, limit=64 << 20):
+    """The per-gene tables and trend record one pass of `ResidentFit.run` hands its caller, as float64 .npy files (a few MB at the
+    headline workload).  Above `limit` bytes the per-gene tables keep a fixed, seeded sample of genes, listed in gene_index.npy."""
+    scalars = {"prior_var": res["prior_var"], "squared_logres": res["squared_logres"], "trend_coeffs": res["trend"].coeffs}
+    per_gene = {k: np.asarray(v, dtype=np.float64) for k, v in res.items() if k not in scalars and k != "trend"}
+    G = len(res["dispersions"])
+    row_bytes = sum(a.nbytes for a in per_gene.values()) // max(G, 1)
+    if G * row_bytes > limit:
+        keep = (limit - (1 << 16)) // (row_bytes + 8)  # + gene_index, and room for the .npy headers and the scalars
+        idx = np.sort(np.random.default_rng(0).choice(G, keep, replace=False))
+        per_gene = {k: a[idx] for k, a in per_gene.items()}
+        per_gene["gene_index"] = idx.astype(np.float64)
+    arrays = {**per_gene, **{k: np.atleast_1d(np.asarray(v, dtype=np.float64)) for k, v in scalars.items()}}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def make_workload(samples, genes, design, rank, dist=None):
@@ -162,7 +189,7 @@ def run_reference(args, rank, world):
     cpu_fit(sample[:, :256], X, sf, cores)  # spawn the loky pool outside the timed region
     for _ in range(max(1, min(args.warmup, 2))):
         cpu_fit(sample, X, sf, cores)
-    steps = max(1, min(args.steps, 5))  # bounded: the arm must end within minutes (one pass is ~6 s on 128 cores)
+    steps = args.steps
     times = [cpu_fit(sample, X, sf, cores) for _ in range(steps)]
     dt = float(np.median(times))
     val = n_in / dt
@@ -293,7 +320,7 @@ class Bench:
         for _ in range(steps):
             self.flush_l2()
             self.barrier()
-            rf.run(events=(0, 1))  # CUDA events around the device work of the pass: first launch ... result copy done
+            out = rf.run(events=(0, 1))  # CUDA events around the device work of the pass: first launch ... result copy done
             step_ms.append(self.ctx.elapsed_ms(0, 1))
         self.barrier()
         launches = self.ctx.launches() - launches0
@@ -306,7 +333,7 @@ class Bench:
         if self.world > 1:  # how the shards exchanged: peer-memory push kernel (NVLink stores) or grouped NCCL all-gathers
             rec["exchange"] = "peer" if rf._win is not None else "nccl"
         rec.update(self.rooflines(stages, N, G, X.shape[1], ms))
-        return rf, rec
+        return rf, rec, out
 
     def rooflines(self, stages, N, G, p, step_ms):
         """HBM roofline of the dominant kernel and of the whole step; FP64 roofline of the dominant kernel (DFMA peak measured in
@@ -449,12 +476,14 @@ def main():
 
     # ---------------------------------------------------------------- value: device-resident (headline workload)
     clk = ClockSampler(B.local).__enter__()  # sampled from the warm-up until the end of the e2e loop (steps last only ms)
-    rf, head = B.resident(counts, X, sf, G_in, args.steps, args.warmup)
+    rf, head, last_out = B.resident(counts, X, sf, G_in, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last_out)
     stages = dict(head["stages_ms"])
     shard_check = B.check_shards(rf) if world > 1 else None
     exchange_ab = None
     if world > 1 and head.get("exchange") == "peer":  # the same steps with the NCCL exchange, for comparison
-        rf_n, rec_n = B.resident(counts, X, sf, G_in, args.steps, args.warmup, exchange="nccl")
+        rf_n, rec_n, _ = B.resident(counts, X, sf, G_in, args.steps, args.warmup, exchange="nccl")
         rf_n.close()
         exchange_ab = {"peer_ms_per_step": head["ms_per_step"], "nccl_ms_per_step": rec_n["ms_per_step"],
                        "nccl_stages_ms": {k: rec_n["stages_ms"][k] for k in ("allgather", "gather_results") if k in rec_n["stages_ms"]}}
@@ -483,12 +512,12 @@ def main():
 
     # ---------------------------------------------------------------- e2e: plugin calls with host buffers
     e2e = B.e2e(counts, X, sf, G_in, args.steps, pinned=True)
-    e2e_pageable = B.e2e(counts, X, sf, G_in, max(2, min(args.steps, 5)), pinned=False)
+    e2e_pageable = B.e2e(counts, X, sf, G_in, args.steps, pinned=False)
     e2e["pageable"] = e2e_pageable
     time.sleep(0.25)  # let nvidia-smi emit at least one more sample
     clk.__exit__()
 
-    full = B.full_deseq2(counts, X, sf, G_in, max(3, min(args.steps, 10))) if world == 1 else None
+    full = B.full_deseq2(counts, X, sf, G_in, args.steps) if world == 1 else None
 
     # ---------------------------------------------------------------- BASELINE's larger shapes, same measurement
     configs = {}
@@ -499,13 +528,13 @@ def main():
             extra.insert(0, ("C3", 60000, 500, "factorial", "BASELINE.json configs[2]: 60 000 genes x 500 samples, 3 covariates, whole on one GPU"))
         for name, g, n, design, what in extra:
             c2, X2, sf2, gin2 = make_workload(n, g, design, rank, B.dist)
-            rf2, rec = B.resident(c2, X2, sf2, gin2, max(3, min(args.steps, 10)), 3)
+            rf2, rec, _ = B.resident(c2, X2, sf2, gin2, args.steps, 3)
             rec["workload"] = f"{what}; {g} genes x {n} samples per GPU, {design} design (p={P_OF[design]})"
             if world > 1:
                 rec["shard_check"] = B.check_shards(rf2)
             rf2.close()
             if name == "C3":
-                rec["e2e"] = B.e2e(c2, X2, sf2, gin2, 3, pinned=True)
+                rec["e2e"] = B.e2e(c2, X2, sf2, gin2, args.steps, pinned=True)
             configs[name] = rec
             del c2, rf2
 

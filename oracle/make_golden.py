@@ -511,6 +511,9 @@ def main_grid_beta():
 
 
 if __name__ == "__main__":
+    from oracle import build_ref
+
+    build_ref.build()  # the shim imports the reference package from its byte-compiled copy
     if len(sys.argv) > 1 and sys.argv[1] == "grid_beta":
         main_grid_beta()
     elif len(sys.argv) > 1 and sys.argv[1] == "e2e":  # end-to-end fixtures only

@@ -1,12 +1,11 @@
-"""Import shim (TEST INFRASTRUCTURE, container-only).
+"""Import shim (TEST INFRASTRUCTURE).
 
-Makes the read-only reference checkout at /root/reference importable without
-installing it: the real ``pydeseq2/__init__.py`` calls
-``importlib.metadata.version("pydeseq2")`` which fails for an un-installed tree.
-Only used by ``oracle/make_golden.py`` and the ``refcheck`` tests that run in the
-build container; nothing on the product path imports it and it is never present on
-the GPU box (``/root/reference`` does not exist there).
+Makes the reference package importable without installing it, from the byte-compiled copy ``build()`` leaves in
+``oracle/_ref/pydeseq2`` (oracle/build_ref.py): the real ``pydeseq2/__init__.py`` calls
+``importlib.metadata.version("pydeseq2")``, which fails for an un-installed tree, so this module stands in for it.
+Only used by ``oracle/make_golden.py`` and the drop-in tests; nothing on the product path imports it.
 """
-__path__ = ["/root/reference/pydeseq2"]
-__file__ = "/root/reference/pydeseq2/__init__.py"
+import os as _os
+
+__path__ = [_os.path.join(_os.path.dirname(_os.path.dirname(_os.path.dirname(_os.path.abspath(__file__)))), "_ref", "pydeseq2")]
 __version__ = "0.5.3"

@@ -14,7 +14,7 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box via gpurun)")
-    config.addinivalue_line("markers", "refcheck: needs the read-only reference checkout at /root/reference")
+    config.addinivalue_line("markers", "refcheck: needs the reference package build() byte-compiles into oracle/_ref")
 
 
 def load_golden(name):

@@ -1,6 +1,6 @@
-"""Helper of tests/test_reference_dropin.py, run in a SUBPROCESS (build container only): the REAL, unmodified orchestrator of the
+"""Helper of tests/test_reference_dropin.py, run in a SUBPROCESS: the REAL, unmodified orchestrator of the
 reference (`DeseqDataSet.deseq2()`, `DeseqStats.summary()`, `lfc_shrink()`) with `B200Inference` injected as its `inference=`
-backend -- device algorithms through the host emulator, since this container has no GPU.  Writes the final tables to an .npz.
+backend -- device algorithms through the host emulator, so no GPU is needed.  Writes the final tables to an .npz.
 The import shims (oracle/refshim*) stay inside this process."""
 import os
 import sys

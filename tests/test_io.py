@@ -6,9 +6,11 @@ import numpy as np
 import pandas as pd
 import pytest
 
+from conftest import GOLDEN
 from pydeseq2_b200.io import read_counts_csv
 
-REF = "/root/reference/datasets/synthetic/test_counts.csv"
+# the reference's shipped synthetic dataset (datasets/synthetic/test_counts.csv), stored as is
+REF = os.path.join(GOLDEN, "synthetic_test_counts.csv")
 
 
 def _write(path, df, **kw):
@@ -55,8 +57,6 @@ def test_ragged_line_is_rejected(tmp_path):
         read_counts_csv(p)
 
 
-@pytest.mark.refcheck
-@pytest.mark.skipif(not os.path.exists(REF), reason="reference checkout not present")
 def test_reference_shipped_dataset():
     want = pd.read_csv(REF, index_col=0).T
     got = read_counts_csv(REF)

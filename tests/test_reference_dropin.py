@@ -1,6 +1,6 @@
-"""CPU suite, build container only: `B200Inference` plugged into the REAL reference orchestrator (`DeseqDataSet(..., inference=)`,
+"""CPU suite: `B200Inference` plugged into the REAL reference orchestrator (`DeseqDataSet(..., inference=)`,
 `DeseqStats(..., inference=)`), i.e. the drop-in claim of INTEGRATION.md exercised with the reference's own objects.  The device
-algorithms run through the host emulator.  Skipped where the read-only checkout is absent (the GPU box)."""
+algorithms run through the host emulator.  The reference package is the byte-compiled copy build() leaves in oracle/_ref."""
 import os
 import subprocess
 import sys
@@ -11,8 +11,10 @@ import pytest
 from conftest import GOLDEN, load_golden
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+REF_PKG = os.path.join(os.path.dirname(HERE), "oracle", "_ref", "pydeseq2")
 pytestmark = [pytest.mark.refcheck,
-              pytest.mark.skipif(not os.path.isdir("/root/reference/pydeseq2"), reason="needs the reference checkout")]
+              pytest.mark.skipif(not os.path.isfile(os.path.join(REF_PKG, "dds.pyc")),
+                                 reason="the reference package was not compiled into oracle/_ref (build() found no reference checkout)")]
 
 
 @pytest.mark.parametrize("name,mode", [("e2e_two_level_n24", "plugin"), ("e2e_factorial_n20", "plugin"),
